@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — SA-SSD inference hot path on B200: frames/sec on synthetic KITTI-shaped clouds.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the whole hot path (voxelize -> anchors_mask -> 13 sparse convs ->
@@ -322,7 +322,18 @@ def parity_check(model, sd, batches, batch, maxpts, n_frames=2):
     return res
 
 
-MIN_TIMED_S = 1.0      # the timed region repeats the K steps until it is at least this long
+def dump_outputs(out_dir, det_all, nd_all):
+    """What the timed path returned in its last step, in global frame order: per-frame detection counts and the
+    detections of all frames concatenated (boxes_lidar [D, 7], scores [D], label_preds [D]).  Rows past a frame's
+    count are scratch and are left out, so that two builds can be compared array for array."""
+    from sassd_b200 import dist as D
+    det, nd = D.interleave(det_all, nd_all)
+    det, nd = det.cpu().numpy(), nd.cpu().numpy()
+    rows = np.concatenate([det[f, :int(nd[f])] for f in range(det.shape[0])], 0)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("num_detections", nd.astype(np.float64)), ("boxes_lidar", rows[:, :7]), ("scores", rows[:, 7]),
+                    ("label_preds", rows[:, 8].astype(np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def run_ours(args, rank, world, local):
@@ -365,22 +376,18 @@ def run_ours(args, rank, world, local):
             return graph.replay() + (None,)
         return model.forward_device(p, o, B, mx)
 
-    t_est0 = time.perf_counter()
     for i in range(max(3, args.warmup)):
         det, nd, status, aux = step(i)
     torch.cuda.synchronize()
-    est_step_s = (time.perf_counter() - t_est0) / max(3, args.warmup)
     word = int(status.item())
     assert word == 0, "device status flags %s" % ops._lib.decode_flags(word)
     # the shard's single exchange step: pre-allocated, warmed before anything is timed
     gather = D.DetectionGather(det.shape[0], det.shape[1], dev)
     gather.warm()
 
-    # ---- timed region: K steps (repeated `rounds` times until >= MIN_TIMED_S), CUDA events on the launching
-    # stream around every step, L2 flushed (untimed) between steps, + the result gather, max over ranks
-    rounds = max(1, int(np.ceil(MIN_TIMED_S / max(args.steps * est_step_s, 1e-6))))
-    rounds = int(D.max_over_ranks(rounds, dev))
-    nsteps = args.steps * rounds
+    # ---- timed region: K steps, CUDA events on the launching stream around every step, L2 flushed (untimed) between
+    # steps, + the result gather, max over ranks
+    nsteps = args.steps
     sampler = ClockSampler(local)
     D.barrier(); torch.cuda.synchronize()
     sampler.start()
@@ -404,6 +411,8 @@ def run_ours(args, rank, world, local):
     D.barrier(); torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_wall0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:      # before anything reuses the graph's or the gather's output buffers
+        dump_outputs(args.dump_outputs, det_all, nd_all)
     launches = (ops.LAUNCHES - l0)
     if graph is not None:      # launches are inside the captured graph: count the kernels of one eager step
         l1 = ops.LAUNCHES
@@ -550,15 +559,15 @@ def run_ours(args, rank, world, local):
                           "rotated NMS)" % nsamp)
 
     line = dict(metric=METRIC, value=value, unit="frames/s", n_gpus=world, steps=args.steps, warmup=max(3, args.warmup),
-                ms_per_step=dev_ms / nsteps, steps_timed=nsteps, rounds=rounds, higher_is_better=True, scaling="weak",
+                ms_per_step=dev_ms / nsteps, steps_timed=nsteps, higher_is_better=True, scaling="weak",
                 vs_baseline=None, dtype="f32", data="synthetic", impl="ours", config=workload_config(B),
                 details=dict(weights="synthetic (seed 0, BN calibrated)",
                              l2="flushed between steps (256 MiB memset, untimed)", precision=args.precision,
                              bev_tile_skipping=bool(ops.TILE_OCCUPANCY), sparse_tap_skipping=bool(ops.SPCONV_TAP_SKIP),
                              sparse_tap_split=bool(ops.SPCONV_TAP_SPLIT), cuda_graph=graph is not None,
                              parallelism="frames sharded, dp%d" % world,
-                             timed_region="%d x %d steps (>= %.1f s), per-step CUDA events + the result all_gather "
-                                          "(%.3f ms)" % (rounds, args.steps, MIN_TIMED_S, gather_ms)),
+                             timed_region="%d steps, per-step CUDA events + the result all_gather (%.3f ms)"
+                                          % (nsteps, gather_ms)),
                 clocks=clocks, gpu_launches=launches,
                 e2e=dict(value=e2e, unit="frames/s", h2d_bytes_per_step=h2d, d2h_bytes_per_step=d2h,
                          api="SingleStageDetector.detect_stream (host numpy points in, numpy detections out) + the "
@@ -751,7 +760,13 @@ def main():
     ap.add_argument("--serial-stream", action="store_true",
                     help="e2e: one step on the GPU at a time (default: detect_stream keeps --in-flight captured steps going)")
     ap.add_argument("--in-flight", type=int, default=4, help="captured steps detect_stream keeps in flight (e2e)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the detections of the last timed step as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     WORKLOAD.update(config=args.config, density=args.density)
     from sassd_b200 import dist as D
     if args.impl == "reference":

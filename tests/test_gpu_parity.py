@@ -5,7 +5,6 @@ golden fixtures produced by the reference's own Python.
 Bar: bit-exact for voxel indices, rulebooks, anchors masks and NMS keep masks; fp32
 feature / score / box tolerances are written next to each assertion.
 """
-import ctypes
 import os
 
 import numpy as np
@@ -335,42 +334,38 @@ def _random_boxes(n, seed, spread=20.0):
     return b7, s
 
 
-def _load_ref_nms():
-    from oracle import build as ob
-    path = ob.build_ref()
-    if path is None:
-        return None
-    lib = ctypes.CDLL(path)
-    fn = getattr(lib, "_Z11nmsLauncherPKfPyif")
-    fn.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_float]
-    fn.restype = None
-    return fn
+NMS_CASES = [(1, 0), (2, 1), (63, 2), (64, 3), (65, 4), (300, 5), (1500, 6)]
+NMS_THR = 0.1
 
 
-@pytest.mark.parametrize("n,seed", [(1, 0), (2, 1), (63, 2), (64, 3), (65, 4), (300, 5), (1500, 6)])
-def test_nms_mask_and_keep(dev, n, seed):
-    """Keep mask vs the CPU oracle; suppression bitmask vs the UNMODIFIED reference CUDA kernel
-    (oracle/_ref, built from /root/reference in the build container) bit for bit."""
-    from sassd_b200 import ops
-    from sassd_b200.single_stage_heads import boxes3d_to_bev_torch, nms_gpu
+def nms_case(n, seed):
+    """Scores and BEV boxes [n, 5] of one NMS case, and the boxes sorted by descending score (the kernels' input)."""
+    from sassd_b200.single_stage_heads import boxes3d_to_bev_torch
     b7, s = _random_boxes(n, seed)
     bev = boxes3d_to_bev_torch(torch.from_numpy(b7))
     order = torch.sort(torch.from_numpy(s), descending=True, stable=True)[1]
-    sorted_bev = bev[order].contiguous()
-    thr = 0.1
+    return s, bev, bev[order].contiguous()
+
+
+@pytest.mark.parametrize("n,seed", NMS_CASES)
+def test_nms_mask_and_keep(dev, golden_dir, n, seed):
+    """Keep mask vs the CPU oracle; suppression bitmask bit for bit vs the one the UNMODIFIED reference CUDA kernel
+    computed on the same boxes (tests/golden/nms.npz, made by tests/golden/make_golden_nms.py)."""
+    from sassd_b200 import ops
+    from sassd_b200.single_stage_heads import nms_gpu
+    s, bev, sorted_bev = nms_case(n, seed)
+    thr = NMS_THR
     mask = ops.nms_mask(sorted_bev.to(dev), thr).cpu().numpy().view(np.uint64)
-    ref = _load_ref_nms()
     colb = (n + 63) // 64
     upper = np.zeros((n, colb), bool)
     for i in range(n):
         upper[i, i // 64:] = True
-    if ref is not None:
-        rmask = torch.zeros((n, colb), dtype=torch.int64, device=dev)
-        torch.cuda.synchronize()
-        ref(ctypes.c_void_p(sorted_bev.to(dev).data_ptr()), ctypes.c_void_p(rmask.data_ptr()), n, ctypes.c_float(thr))
-        torch.cuda.synchronize()
-        rm = rmask.cpu().numpy().view(np.uint64)
-        assert np.array_equal(mask[upper], rm[upper]), "suppression bitmask differs from the reference kernel"
+    g = np.load(os.path.join(golden_dir, "nms.npz"))
+    key = "n%d_seed%d" % (n, seed)
+    assert np.array_equal(sorted_bev.numpy(), g[key + "_bev"]), "the boxes differ from those the reference kernel saw"
+    rm = g[key + "_mask"]
+    assert rm.shape == mask.shape
+    assert np.array_equal(mask[upper], rm[upper]), "suppression bitmask differs from the reference kernel"
     keep = nms_gpu(bev.to(dev), torch.from_numpy(s).to(dev), thr).cpu().numpy()
     okeep = O.nms_rotated(bev, torch.from_numpy(s), thr).numpy()
     iou = O.iou_matrix(sorted_bev.numpy())

@@ -1,5 +1,6 @@
 """CPU-side tests: host logic, the C-ABI library's exports, checkpoint format, config loader."""
 import ctypes
+import json
 import os
 import re
 
@@ -81,13 +82,20 @@ def test_config_loader_and_registry():
         S.Config.fromfile("/nonexistent.py")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/configs"), reason="reference tree only in the build container")
-def test_reference_configs_load_unchanged():
+def test_reference_configs_load_unchanged(golden_dir):
+    """The reference's two configs as Config.fromfile parsed them (tests/golden/reference_configs.json, made by
+    tests/golden/make_golden_configs.py) build unchanged, and the project's configs hold the same values."""
     import sassd_b200 as S
+    with open(os.path.join(golden_dir, "reference_configs.json")) as f:
+        ref = json.load(f)
     for name, na in (("car_cfg.py", 70400), ("multi_cfg.py", 211200)):
-        cfg = S.Config.fromfile(os.path.join("/root/reference/configs", name))
+        cfg = S.Config(ref[name])
         model, vg, aset = S.build_from_config(cfg, device="cpu")
         assert aset.anchors.shape[0] == na
+        ours = json.loads(json.dumps(S.Config.fromfile(os.path.join(ROOT, "configs", name))._cfg_dict))
+        assert ours["model"] == ref[name]["model"] and ours["test_cfg"] == ref[name]["test_cfg"], name
+        for k, v in ref[name]["data"]["val"].items():
+            assert ours["data"]["val"][k] == v, (name, k)
 
 
 def test_checkpoint_roundtrip_reference_format(tmp_path):

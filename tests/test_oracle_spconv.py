@@ -89,7 +89,9 @@ def test_indice_pairs_canonical_form():
 
 
 def test_vxnet_tiny_end_to_end_vs_dense():
-    """Whole VxNet on a tiny grid vs a dense conv3d network with active-site masking."""
+    """Whole VxNet on a tiny grid vs a dense conv3d network with active-site masking.  The dense emulation runs in
+    float64: in fp32 its own summation order, which depends on the host's CPU kernels and thread count, uses up to
+    1.2x of the tolerance on these 14 layers, so the tolerance is left to the fp32 oracle alone."""
     from sassd_b200.checkpoint import make_synthetic_state_dict
     sd = make_synthetic_state_dict(seed=3, num_class=1)
     B, shape = 1, [8, 16, 16]
@@ -97,22 +99,23 @@ def test_vxnet_tiny_end_to_end_vs_dense():
     feats, c3, shape3 = O.vxnet_forward(sd, f, c, shape)
     assert shape3 == [1, 2, 2] and feats.shape[1] == 64
     # dense emulation
-    x = _densify(c, f, B, shape)
+    sd64 = {k: (v.double() if v.is_floating_point() else v) for k, v in sd.items()}
+    x = _densify(c, f, B, shape).double()
     act = _densify(c, torch.ones(c.shape[0], 1), B, shape) > 0
     p = "neck.backbone."
 
     def bnrelu(x, name):
-        return torch.relu(O.bn_eval(x, sd, p + name))
+        return torch.relu(O.bn_eval(x, sd64, p + name))
     for block, idxs, kind, key in O.VXNET_PLAN:
         for i in idxs:
-            w = sd["%s%s.%d.weight" % (p, block, i)].permute(4, 3, 0, 1, 2).contiguous()
+            w = sd64["%s%s.%d.weight" % (p, block, i)].permute(4, 3, 0, 1, 2).contiguous()
             if kind == "down":
                 x = F.conv3d(x, w, stride=2, padding=1)
                 act = F.conv3d(act.float(), torch.ones(1, 1, 3, 3, 3), stride=2, padding=1) > 0
             else:
                 x = F.conv3d(x, w, padding=1)
             x = bnrelu(x, "%s.%d" % (block, i + 1)) * act
-    w = sd[p + "extra_conv.0.weight"].permute(4, 3, 0, 1, 2).contiguous()
+    w = sd64[p + "extra_conv.0.weight"].permute(4, 3, 0, 1, 2).contiguous()
     x = bnrelu(F.conv3d(x, w), "extra_conv.1") * act
     ci = torch.from_numpy(c3.astype(np.int64))
     ref = x[ci[:, 0], :, ci[:, 1], ci[:, 2], ci[:, 3]]
