@@ -179,8 +179,14 @@ int sassd_gconv_pack(const float* weight, int taps, int cin, int cout, int preci
  * BEVNet / head convolutions (cmn.py:264-282, ssd_rotate_head.py:218-231,424-429) with the activation operand
  * moved by TMA (cp.async.bulk.tensor) instead of producer warps.  A split map is two fp16 planes
  * [2][batch][H][W][C] (C % 64 == 0): hi = half(x), lo = half((x - hi) * 2048).  Outputs: fp32 NHWC
- * (out_f32, stride out_f32_stride) and/or the next layer's split map (out_split, out_split_ch channels, the
- * channels beyond cout written as zero).  wpack: sassd_gconv_pack(..., SASSD_PREC_F16X3).  16 < cout <= 256. */
+ * (out_f32, stride out_f32_stride) and/or the next layer's split map (out_split, out_split_ch channels).
+ * wpack: sassd_gconv_pack(..., SASSD_PREC_F16X3).  16 < cout <= 256.  The stored input channels [cin, cin_stored)
+ * must be zero.  What is written, per pixel of the map: the kernel computes N = cout rounded up to 32, 64, 128 or
+ * 256 channels; of each output it writes channels [0, min(N, width)) (width = out_f32_stride or out_split_ch),
+ * channels [cout, min(N, width)) as +0.0, and leaves channels [N, width) and all memory outside the buffers
+ * untouched - a split map read as the next layer's input with out_split_ch > N must be zeroed beforehand.  Both
+ * outputs carry the same values (the split one is the split of the fp32 one) and do not depend on which outputs
+ * are requested, on tile_order or on n_split. */
 typedef struct {
     int32_t batch, H, W;
     int32_t cin, cin_stored;       /* valid / stored input channels */
@@ -220,7 +226,11 @@ int sassd_sparse_to_bev_split(const float* feat, const int32_t* coors, const int
 /* Ruled sparse conv on "split rows" (two fp16 planes [2][rows][C], C % 8 == 0; hi = half(x), lo = half((x-hi)*2048)):
  * same semantics as sassd_gconv TABLE / ROWS mode with SASSD_PREC_F16X3, but the gather is 16-byte cp.async copies
  * straight into the tensor-core operand tiles and the epilogue writes the next layer's planes (out_split, out_ch
- * channels, zero beyond cout) and/or fp32 rows.  taps == 1: row(m) = m.  cin <= 64, cout <= 64. */
+ * channels) and/or fp32 rows.  taps == 1: row(m) = m.  cin <= 64, cout <= 64.  Only rows m < min(*d_rows, rows_cap)
+ * are written; rows beyond them and all memory outside the buffers are left untouched.  The kernel computes N = cout
+ * rounded up to 16, 32 or 64 channels; of each row it writes channels [0, min(N, width)) (width = out_ch or
+ * out_f32_stride, rounded down to whole 8 / 4-channel groups), channels [cout, min(N, width)) as +0.0, and leaves
+ * channels [N, width) untouched. */
 typedef struct {
     int32_t cin, cout, taps;         /* cin = stored channels of the input planes */
     int32_t rows_cap, in_rows_cap;   /* output rows capacity; rows of the input planes (plane stride) */
@@ -243,7 +253,8 @@ int sassd_spconv_f16x3(const sassd_spconv_desc* host_desc, const void* in_split,
                        const float* shift, const int32_t* nbr, const int32_t* tile_mask, const int32_t* d_rows,
                        void* out_split, float* out_f32, void* ws, size_t ws_bytes, int32_t* counters,
                        sassd_stream_t stream);
-/* fp32 rows [rows, cin] -> split rows [2][rows_cap][cs] (cs >= cin, cs % 8 == 0, padding zero). */
+/* fp32 rows [rows, cin] -> split rows [2][rows_cap][cs] (cs >= cin, cs % 8 == 0, padding channels +0.0).  Rows at or
+ * beyond *d_rows (d_rows == NULL: rows_cap) are not written. */
 int sassd_features_to_split(const float* feat, const int32_t* d_rows, int rows_cap, int cin, int cs, void* out_split,
                             sassd_stream_t stream);
 /* dense() of split rows into a (pre-zeroed) split BEV map [2,batch,H,W,D*C]. */

@@ -1,5 +1,5 @@
-"""GPU dev tool: check the tcgen05 (3xTF32) gathered-GEMM kernel against the FFMA path and fp64,
-smallest cases first, printing diagnostics instead of asserting."""
+"""GPU dev tool: timings and traces of the tensor-core conv kernels at pipeline shapes (each timed case also prints
+its error against fp64).  The kernel-level correctness checks live in tests/test_conv_kernels.py."""
 import os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
@@ -83,26 +83,6 @@ def run(mode, M, cin, cout, taps, relu, H=0, W=0, B=0, nbr=None, d_rows=None, ta
 
 
 stage = sys.argv[1] if len(sys.argv) > 1 else "all"
-if stage in ("tiny", "all"):
-    run(ops.GCONV_ROWS, 128, 32, 16, 1, False, tag="rows tiny pattern", pattern="ones")
-    run(ops.GCONV_ROWS, 128, 32, 16, 1, False, tag="rows tiny")
-    run(ops.GCONV_ROWS, 128, 32, 64, 1, True, tag="rows 1 tile N64")
-    run(ops.GCONV_ROWS, 128, 64, 256, 1, True, tag="rows 1 tile N256 2 chunks")
-    run(ops.GCONV_ROWS, 1000, 256, 256, 1, True, tag="rows multi-tile")
-    run(ops.GCONV_ROWS, 1000, 28, 28, 1, False, tag="rows cin=28 (K tail) cout=28")
-    run(ops.GCONV_ROWS, 777, 256, 20, 1, False, tag="rows 256->20")
-if stage in ("conv", "all"):
-    run(ops.GCONV_CONV2D, 2 * 12 * 10, 32, 16, 9, True, H=12, W=10, B=2, tag="conv2d small")
-    run(ops.GCONV_CONV2D, 1 * 40 * 36, 256, 256, 9, True, H=40, W=36, B=1, tag="conv2d 256->256 40x36")
-    run(ops.GCONV_CONV2D, 1 * 40 * 36, 320, 256, 9, True, H=40, W=36, B=1, tag="conv2d 320->256 40x36")
-    run(ops.GCONV_CONV2D, 1 * 40 * 36, 256, 28, 9, True, H=40, W=36, B=1, tag="conv2d 256->28 40x36")
-if stage in ("table", "all"):
-    rs = np.random.RandomState(0)
-    for cin, cout in ((4, 16), (16, 16), (16, 32), (32, 64), (64, 64)):
-        M = 3000
-        nbr = torch.from_numpy(np.where(rs.rand(M, 27) < 0.3, rs.randint(0, M, (M, 27)), -1).astype(np.int32)).to(dev)
-        d_rows = torch.tensor([M - 37], dtype=torch.int32, device=dev)
-        run(ops.GCONV_TABLE, M, cin, cout, 27, True, nbr=nbr, d_rows=None, tag="table %d->%d" % (cin, cout))
 if stage in ("perf", "all"):
     run(ops.GCONV_CONV2D, 200 * 176, 256, 256, 9, True, H=200, W=176, B=1, tag="BEV 3x3 256->256 B=1", time_it=True)
     run(ops.GCONV_CONV2D, 4 * 200 * 176, 256, 256, 9, True, H=200, W=176, B=4, tag="BEV 3x3 256->256 B=4", time_it=True)
@@ -147,14 +127,6 @@ def run_tma(B, H, W, cin, cout, taps, relu, tag, time_it=False):
         print("   tma f16x3 %.3f ms  %.1f TFLOP/s (algorithmic fp32)" % (ms, 2.0 * B * H * W * cin * cout * taps / ms / 1e9), flush=True)
 
 
-if stage in ("tma", "all"):
-    run_tma(1, 8, 16, 64, 32, 1, False, "tma 1 tile 1x1")
-    run_tma(1, 8, 16, 64, 32, 9, True, "tma 1 tile 3x3")
-    run_tma(2, 24, 20, 256, 256, 9, True, "tma 256->256 partial tiles")
-    run_tma(1, 40, 36, 320, 256, 9, True, "tma 320->256")
-    run_tma(1, 40, 36, 256, 28, 9, True, "tma 256->28")
-    run_tma(1, 40, 36, 28, 28, 1, False, "tma 28->28 1x1")
-    run_tma(1, 40, 36, 256, 20, 1, False, "tma 256->20 1x1")
 if stage in ("tmaperf", "all"):
     run_tma(1, 200, 176, 256, 256, 9, True, "tma BEV 3x3 B=1", time_it=True)
     run_tma(4, 200, 176, 256, 256, 9, True, "tma BEV 3x3 B=4", time_it=True)
@@ -182,74 +154,6 @@ def tile_masks(nb, n_rows):
     return (present * (1 << np.arange(taps))[None, :]).sum(1).astype(np.int32)
 
 
-def run_split(M, cin, cout, taps, relu, tag, density=0.3, masks=False, absent=0.0):
-    """masks: pass the per-tile tap masks (tap skipping); absent: fraction of (tile, tap) combinations with no
-    neighbour at all, so that whole chunks really are skipped."""
-    rs = np.random.RandomState(cin * 100 + cout)
-    x = torch.randn(M, cin, device=dev)
-    w = torch.randn(taps, cin, cout, device=dev) * 0.1
-    scale = torch.rand(cout, device=dev) + 0.5
-    shift = torch.randn(cout, device=dev) * 0.1
-    nbr = tm = None
-    if taps > 1:
-        nb = np.where(rs.rand(M, taps) < density, rs.randint(0, M, (M, taps)), -1).astype(np.int32)
-        if absent > 0:
-            gone = rs.rand((M + 127) // 128, taps) < absent
-            gone[0, :] = True        # a tile with no pair at all must still produce act(shift)
-            nb[np.repeat(gone, 128, axis=0)[:M]] = -1
-        nbr = torch.from_numpy(nb).to(dev)
-        if masks:
-            tm = torch.from_numpy(tile_masks(nb, M - 5)).to(dev)
-    d_rows = torch.tensor([M - 5], dtype=torch.int32, device=dev)
-    planes = ops.features_to_split(x)
-    out, of = ops.spconv_split(planes, w, scale, shift, relu, cout, M, nbr=nbr, d_rows=d_rows, want_f32=True,
-                               tile_mask=tm)
-    torch.cuda.synchronize()
-    xd, wd = x.double().cpu(), w.double().cpu()
-    ref = torch.zeros(M, cout, dtype=torch.float64)
-    if taps == 1:
-        ref = xd @ wd[0]
-    else:
-        nb = nbr.cpu().long()
-        for t in range(taps):
-            o = torch.nonzero(nb[:, t] >= 0).view(-1)
-            ref.index_add_(0, o, xd[nb[o, t]] @ wd[t])
-    ref = ref * scale.double().cpu() + shift.double().cpu()
-    if relu:
-        ref = ref.clamp_min(0)
-    n = M - 5
-    sc = ref.abs().max().item()
-    e1 = (of[:n, :cout].double().cpu() - ref[:n]).abs().max().item()
-    e2 = (ops.split_rows_float(out, cout)[:n].double().cpu() - ref[:n]).abs().max().item()
-    ok = e1 < 2e-5 * max(sc, 1) and e2 < 2e-5 * max(sc, 1)
-    print("%-26s M=%-6d cin=%-3d cout=%-3d taps=%-2d |ref|max %.3g  err f32 %.2e  err split %.2e  %s" %
-          (tag, M, cin, cout, taps, sc, e1, e2, "OK" if ok else "MISMATCH"), flush=True)
-    if not ok:
-        d = (of[:n, :cout].double().cpu() - ref[:n]).abs()
-        bad = torch.nonzero(d > 1e-3 * max(sc, 1))
-        print("   n_bad", bad.shape[0], "first", bad[:6].tolist())
-        print("   got", of[0, :6].tolist(), "ref", ref[0, :6].tolist())
-
-
-if stage in ("split",):
-    run_split(128, 8, 16, 1, False, "split rows 1 tile")
-    run_split(300, 4, 16, 27, True, "split table 4->16")
-    run_split(3000, 16, 16, 27, True, "split table 16->16")
-    run_split(3000, 16, 32, 27, True, "split table 16->32")
-    run_split(3000, 32, 64, 27, True, "split table 32->64")
-    run_split(3000, 64, 64, 27, True, "split table 64->64")
-    run_split(20000, 64, 64, 27, True, "split table 64->64 big")
-    run_split(3000, 64, 64, 1, True, "split rows 64->64")
-    # tap skipping (tile masks) with whole (tile, tap) combinations absent; <= 74 tiles also take the cluster tap split
-    run_split(300, 4, 16, 27, True, "skip 4->16", masks=True, absent=0.5)
-    run_split(3000, 16, 32, 27, True, "skip 16->32", masks=True, absent=0.5)
-    run_split(3000, 32, 32, 27, True, "skip 32->32", masks=True, absent=0.4)
-    run_split(3000, 64, 64, 27, True, "skip 64->64 (tap split)", masks=True, absent=0.4)
-    run_split(9400, 64, 64, 27, True, "skip 64->64 74 tiles", masks=True, absent=0.4)
-    run_split(9500, 64, 64, 27, True, "skip 64->64 75 tiles", masks=True, absent=0.4)
-    run_split(20000, 64, 64, 27, True, "skip 64->64 big", masks=True, absent=0.4)
-    run_split(20000, 64, 64, 27, True, "skip 64->64 big sparse", masks=True, absent=0.9, density=0.5)
-    print("done split")
 if stage in ("splitperf",):
     M, cin, cout, taps = 120000, 64, 64, 27
     rs = np.random.RandomState(1)
