@@ -299,6 +299,10 @@ int sassd_pswarp(const float* feat, int feat_stride, int batch, int H, int W, co
  * iou3d.cpp:73-120, iou3d_kernel.cu:250-292) with the greedy sweep on the
  * device, gather.  Sort is stable (score descending, then candidate order).
  * det [batch,det_cap,9] = (x,y,z,w,l,h,ry,score,label); d_ndet [batch].
+ * Per frame the candidates are rows [0, min(d_k, k_cap)); rows beyond are not read.  More than nms_cap passing
+ * candidates: the first nms_cap of them in candidate order go on (not the best-scoring ones), SASSD_FLAG_NMS_CAP.
+ * More than det_cap kept boxes: det holds the first det_cap in score order, SASSD_FLAG_DET_CAP.  det rows at or
+ * beyond d_ndet are not written.
  * ---------------------------------------------------------------------- */
 size_t sassd_rescore_nms_workspace_bytes(int batch, int k_cap, int nms_cap);
 int sassd_rescore_nms(const float* boxes, const float* scores, const int32_t* labels, const int32_t* d_k,
@@ -309,7 +313,8 @@ int sassd_rescore_nms(const float* boxes, const float* scores, const int32_t* la
 /* iou3d_cuda.nms_gpu alone (iou3d.cpp:73-120): boxes [n,5] already sorted by
  * score; mask [n, ceil(n/64)] u64 in the reference layout (only columns j > i
  * are filled; the reference also fills the unused lower triangle); keep [n]
- * int64 indices, *d_nkeep their number. */
+ * int64 indices, *d_nkeep their number.  ws: sassd_nms_workspace_bytes(n) bytes (0 for n == 0, where ws may be
+ * NULL). */
 size_t sassd_nms_workspace_bytes(int n);
 int sassd_nms_mask(const float* boxes5, int n, float thr, uint64_t* mask, sassd_stream_t stream);
 int sassd_nms_sorted(const float* boxes5, int n, float thr, int64_t* keep, int32_t* d_nkeep,

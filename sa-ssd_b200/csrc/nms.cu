@@ -428,8 +428,10 @@ extern "C" int sassd_nms_mask(const float* boxes5, int n, float thr, uint64_t* m
 extern "C" int sassd_nms_sorted(const float* boxes5, int n, float thr, int64_t* keep, int32_t* d_nkeep, void* ws,
                                 size_t ws_bytes, sassd_stream_t stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (!boxes5 || !keep || !d_nkeep || !ws || n < 0) return SASSD_ERR_ARG;
+    if (!boxes5 || !keep || !d_nkeep || n < 0) return SASSD_ERR_ARG;
+    // n == 0 needs no workspace (sassd_nms_workspace_bytes(0) == 0), so ws may be NULL there
     if (n == 0) { cudaMemsetAsync(d_nkeep, 0, 4, stream); return SASSD_OK; }
+    if (!ws) return SASSD_ERR_ARG;
     if (ws_bytes < sassd_nms_workspace_bytes(n)) return SASSD_ERR_WORKSPACE;
     const int colb = (n + 63) / 64;
     if ((size_t)colb * 16 > 40000) return SASSD_ERR_UNSUPPORTED;  // > 160k boxes

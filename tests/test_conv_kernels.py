@@ -16,6 +16,8 @@ import numpy as np
 import pytest
 import torch
 
+from tests.kernel_buffers import SENTINEL, Guarded, _p, _stream, pos_zero, untouched
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -235,43 +237,8 @@ def test_tile_dist_model_matches_definition():
 
 
 # ------------------------------------------------------------------------------------------------------------------
-# GPU helpers: guarded buffers, direct C-ABI launches
+# GPU helpers: direct C-ABI launches into guarded buffers (tests/kernel_buffers.py)
 # ------------------------------------------------------------------------------------------------------------------
-SENTINEL = 0xFF          # every byte of an output allocation before the launch (fp16 / fp32 NaN)
-GUARD = 4096
-
-
-class Guarded:
-    """A tensor inside a larger allocation: GUARD bytes of sentinel before and after it, base 1024-byte aligned
-    (TMA), the whole allocation filled with the sentinel."""
-
-    def __init__(self, shape, dtype, dev):
-        n = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
-        self.raw = torch.full((n + 2 * GUARD + 2048,), SENTINEL, dtype=torch.uint8, device=dev)
-        self.lo = (-self.raw.data_ptr()) % 1024 + GUARD
-        self.hi = self.lo + n
-        self.t = self.raw[self.lo:self.hi].view(dtype).view(shape)
-
-    def guards_intact(self):
-        return bool((self.raw[:self.lo] == SENTINEL).all()) and bool((self.raw[self.hi:] == SENTINEL).all())
-
-
-def untouched(t):
-    return t.numel() == 0 or bool((t.contiguous().view(torch.uint8) == SENTINEL).all())
-
-
-def pos_zero(t):
-    return t.numel() == 0 or bool((t.contiguous().view(torch.uint8) == 0).all())
-
-
-def _p(t):
-    return ctypes.c_void_p(0 if t is None else t.data_ptr())
-
-
-def _stream():
-    return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-
-
 @pytest.fixture(scope="module")
 def dev():
     from sassd_b200 import ops
